@@ -2,6 +2,7 @@
 """bench.py: the headline benchmark -- JSON records/s scanned+aggregated.
 
   python bench.py --gpus N --steps K --warmup W            (our CUDA path)
+      [--dump-outputs DIR]     (+ the last timed step's outputs as .npy)
   python bench.py --impl reference --gpus N --steps K ...  (CPU reference arm)
 
 Workload (BASELINE.json configs[2], the north star's own target shape): 100 M
@@ -29,9 +30,11 @@ learning and the cache lookup a scan does.
 """
 
 import argparse
+import atexit
 import ctypes
 import json
 import os
+import shutil
 import subprocess
 import sys
 import tempfile
@@ -223,6 +226,45 @@ def canon(points):
     return sorted((tuple(repr(c) for c in cols), v) for cols, v in points)
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(d, points, counters):
+    """--dump-outputs: what a caller of the timed scan receives, as float64
+    .npy files under `d`, so that the outputs of two builds can be compared:
+
+      counters.npy      [len(native.COUNTER_FIELDS)], in that order
+      points_count.npy  [n]: each point's count
+      points_key.npy    [n, width]: each point's key as bytes ('s' + the
+                        bytes of a string column, 'n' + repr() of a number,
+                        columns joined by NUL), -1 past its end
+
+    Points are in the order of their key bytes.  Should they come to more
+    than DUMP_LIMIT bytes, a fixed seeded sample of them is written."""
+    import numpy as np
+    from dragnet_b200 import native
+    os.makedirs(d, exist_ok=True)
+    keyed = sorted((b'\0'.join(b's' + c if isinstance(c, bytes)
+                               else b'n' + repr(c).encode() for c in cols), v)
+                   for cols, v in points or [])
+    width = max([len(k) for k, _ in keyed] + [1])
+    cap = max(1, (DUMP_LIMIT - 8 * len(native.COUNTER_FIELDS)) //
+              (8 * (width + 1)))
+    if len(keyed) > cap:
+        pick = np.sort(np.random.default_rng(0).choice(len(keyed), cap,
+                                                       replace=False))
+        keyed = [keyed[i] for i in pick]
+    key = np.full((len(keyed), width), -1.0)
+    for i, (k, _) in enumerate(keyed):
+        key[i, :len(k)] = np.frombuffer(k, dtype=np.uint8)
+    np.save(os.path.join(d, 'points_key.npy'), key)
+    np.save(os.path.join(d, 'points_count.npy'),
+            np.array([v for _, v in keyed], dtype=np.float64))
+    np.save(os.path.join(d, 'counters.npy'),
+            np.array([counters[n] for n in native.COUNTER_FIELDS],
+                     dtype=np.float64))
+
+
 # ---------------------------------------------------------------------------
 # CPU reference arm / cpu_baseline: oracle/ only (no product library)
 # ---------------------------------------------------------------------------
@@ -250,13 +292,28 @@ def run_oracle(plan, path, threads, repeat=1, min_seconds=0.0):
     return json.loads(out)
 
 
+_sample_dir = None
+
+
+def sample_dir():
+    """This run's own directory on tmpfs, removed at exit: samples of another
+    run (another build, another user) are never picked up, and none are left
+    behind."""
+    global _sample_dir
+    if _sample_dir is None:
+        _sample_dir = tempfile.mkdtemp(
+            prefix='dnbench_',
+            dir='/dev/shm' if os.path.isdir('/dev/shm') else None)
+        atexit.register(shutil.rmtree, _sample_dir, True)
+    return _sample_dir
+
+
 def sample_file(rows, seed, total_rows, first=0):
     """Records [first, first + rows) of the `total_rows`-record workload of
     `seed`, written to tmpfs by oracle/gen_ndjson (byte-identical to the device
     generator: tests/test_gpu_parity.py, tests/test_cabi_cpu.py)."""
     _, gen = oracle_build()
-    d = '/dev/shm' if os.path.isdir('/dev/shm') else tempfile.gettempdir()
-    path = os.path.join(d, 'dnbench_sample_%d_%d_%d_%d.ndjson' %
+    path = os.path.join(sample_dir(), 'dnbench_sample_%d_%d_%d_%d.ndjson' %
                         (seed, first, rows, total_rows))
     if not os.path.exists(path):
         subprocess.check_call([gen, path + '.tmp', str(seed), str(total_rows),
@@ -808,6 +865,9 @@ def gpu_arm(args, rank, local_rank, world):
         line['cpu_baseline'] = cpu
     if sampler is not None:
         sampler.stop()
+    if args.dump_outputs:
+        # the last timed step: at N > 1 the merged tallies
+        dump_outputs(args.dump_outputs, R['last'][0], R['last'][1])
     print(json.dumps(line), flush=True)
     if comm is not None:
         L.dng_comm_destroy(comm)
@@ -832,7 +892,14 @@ def main():
     ap.add_argument('--cpu-rows', type=int, default=4000000)
     ap.add_argument('--cpu-seconds', type=float, default=4.0)
     ap.add_argument('--file-steps', type=int, default=2)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the points and counters of the last timed '
+                         'step to DIR as .npy files (see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs: the reference arm scans a different sample')
     rank = int(os.environ.get('RANK', 0))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
