@@ -196,6 +196,10 @@ struct dng_scan {
 	FPlan *d_fplan = nullptr;
 	u8 *d_ftmpl = nullptr;
 	u32 ftmpl_bytes = 0, nftemplates = 0, ftmpl_leaf_off = 0, ftmpl_pool_off = 0;
+	/* dense keys: the value dictionary the compiled matcher was generated
+	 * with (ncols = 0: none), on the device for the end-of-launch flush */
+	FDict fdict{};
+	FDict *d_fdict = nullptr;
 	bool f_kernel = false;
 	u32 f_nt = DNG_F_NT;		/* threads of its CTA: DNG_F_NT, or 768 when
 					 * the tally cache needs the shared memory */
@@ -293,7 +297,8 @@ static void fnt_remember(const dng_scan *s)
 }
 
 int learn_ftemplates(dng_scan *s, const std::vector<TCandidate> &cands,
-    const std::vector<TResolved> &res, size_t sampled_lines)
+    const std::vector<TResolved> &res, size_t sampled_lines, const u8 *head,
+    size_t nhead)
 {
 	std::vector<TResolved> fres(res.size());
 	for (size_t i = 0; i < res.size(); i++)
@@ -314,21 +319,31 @@ int learn_ftemplates(dng_scan *s, const std::vector<TCandidate> &cands,
 	for (size_t i = 0; i < cands.size(); i++)
 		if (accepted[i])
 			covered += cands[i].count;
+	/* the breakdown's values, for the compiled matcher's dense keys */
+	memset(&s->fdict, 0, sizeof (s->fdict));
+	if (s->jit_mode && !blob.empty() && jit_dense())
+		fdict_learn(s->fplan, blob.data(), head, nhead, s->fdict);
 	if (!blob.empty()) {
 		size_t padded = (blob.size() + 127) & ~(size_t)127;
 		blob.resize(padded, 0);
 		CK(s, DEV_ALLOC(s, &s->d_ftmpl, padded));
 		CK(s, cudaMemcpyAsync(s->d_ftmpl, blob.data(), padded,
 		    cudaMemcpyHostToDevice, s->stream));
+		if (s->fdict.ncols) {
+			if (!s->d_fdict)
+				CK(s, DEV_ALLOC(s, &s->d_fdict, sizeof (FDict)));
+			CK(s, cudaMemcpyAsync(s->d_fdict, &s->fdict,
+			    sizeof (FDict), cudaMemcpyHostToDevice, s->stream));
+		}
 		CK(s, cudaStreamSynchronize(s->stream));
 		s->ftmpl_bytes = (u32)padded;
 		s->nftemplates = nt;
 	}
 	s->jit.reset();
 	if (s->jit_mode && !blob.empty())
-		s->jit = jit_request(jit_source(blob.data(), blob.size(), &s->fplan),
-		    (int)s->f_nsl, s->device, (int)s->f_smem_max,
-		    s->jit_mode == 2);
+		s->jit = jit_request(jit_source(blob.data(), blob.size(), &s->fplan,
+		    nullptr, &s->fdict), (int)s->f_nsl, s->device,
+		    (int)s->f_smem_max, s->jit_mode == 2);
 	if (s->kernel_pref == 0)
 		s->f_kernel = s->warp_kernel && !blob.empty() &&
 		    covered * 10 >= sampled_lines * 9 &&
@@ -463,7 +478,8 @@ int learn_templates(dng_scan *s, const u8 *data, unsigned long long start,
 	cached_free(d_res);
 	if (e != cudaSuccess)
 		return s->cuda(e, "template resolve");
-	if (s->fplan.ok && learn_ftemplates(s, cands, res, sampled_lines))
+	if (s->fplan.ok && learn_ftemplates(s, cands, res, sampled_lines,
+	    head.data(), n))
 		return s->err_code;
 	std::vector<u8> blob;
 	u32 nt = 0;
@@ -489,15 +505,18 @@ template <int NSL>
 void launch_fkernel(dng_scan *s, const FScanArgs &a, u32 grid)
 {
 	scan_kernel_f<NSL><<<grid, s->f_nt, fkernel_smem<NSL>(a.tmpl_bytes,
-	    a.s1slots, a.sslots, a.nrows, s->f_nt / 32), s->stream>>>(a);
+	    a.s1slots, a.sslots, a.nrows, s->f_nt / 32, a.ndense),
+	    s->stream>>>(a);
 }
 
-/* tally-cache sizes of the F kernel: what its buffers leave */
+/* tally-cache sizes of the F kernel: what its buffers (and dense counters)
+ * leave */
 template <int NSL>
-void fkernel_slots(const dng_scan *s, u32 nrows, u32 tmpl_room, u32 *s1, u32 *s2)
+void fkernel_slots(const dng_scan *s, u32 nrows, u32 tmpl_room, u32 ndense,
+    u32 *s1, u32 *s2)
 {
 	const size_t fixed = fkernel_smem<NSL>(tmpl_room, 0, 0, nrows,
-	    s->f_nt / 32);
+	    s->f_nt / 32, ndense);
 	const size_t room = s->f_smem_max > fixed ? s->f_smem_max - fixed : 0;
 	u32 n1 = 32;
 	while (n1 < 1024 && (size_t)n1 * 2 * sizeof (SSlot1) +
@@ -570,33 +589,40 @@ int launch_fscan(dng_scan *s, const u8 *data, unsigned long long start,
 	const u32 tmpl_room = jit ? 0 : (u32)TMPL_RESERVE;
 	if (jit)
 		a.tmpl_bytes = 0;
+	/* (dense counters: only the compiled matcher has the dictionary) */
+	a.ndense = jit && s->fdict.ncols ? (s->fdict.total + 3) & ~3u : 0;
+	a.dict = a.ndense ? s->d_fdict : nullptr;
 	size_t smem = 0;
 	switch (nsl) {
 	case 7:
-		fkernel_slots<7>(s, a.nrows, tmpl_room, &a.s1slots, &a.sslots);
+		fkernel_slots<7>(s, a.nrows, tmpl_room, a.ndense, &a.s1slots,
+		    &a.sslots);
 		smem = fkernel_smem<7>(a.tmpl_bytes, a.s1slots, a.sslots, a.nrows,
-		    s->f_nt / 32);
+		    s->f_nt / 32, a.ndense);
 		if (!jit)
 			launch_fkernel<7>(s, a, grid);
 		break;
 	case 9:
-		fkernel_slots<9>(s, a.nrows, tmpl_room, &a.s1slots, &a.sslots);
+		fkernel_slots<9>(s, a.nrows, tmpl_room, a.ndense, &a.s1slots,
+		    &a.sslots);
 		smem = fkernel_smem<9>(a.tmpl_bytes, a.s1slots, a.sslots, a.nrows,
-		    s->f_nt / 32);
+		    s->f_nt / 32, a.ndense);
 		if (!jit)
 			launch_fkernel<9>(s, a, grid);
 		break;
 	case 11:
-		fkernel_slots<11>(s, a.nrows, tmpl_room, &a.s1slots, &a.sslots);
+		fkernel_slots<11>(s, a.nrows, tmpl_room, a.ndense, &a.s1slots,
+		    &a.sslots);
 		smem = fkernel_smem<11>(a.tmpl_bytes, a.s1slots, a.sslots, a.nrows,
-		    s->f_nt / 32);
+		    s->f_nt / 32, a.ndense);
 		if (!jit)
 			launch_fkernel<11>(s, a, grid);
 		break;
 	default:
-		fkernel_slots<13>(s, a.nrows, tmpl_room, &a.s1slots, &a.sslots);
+		fkernel_slots<13>(s, a.nrows, tmpl_room, a.ndense, &a.s1slots,
+		    &a.sslots);
 		smem = fkernel_smem<13>(a.tmpl_bytes, a.s1slots, a.sslots, a.nrows,
-		    s->f_nt / 32);
+		    s->f_nt / 32, a.ndense);
 		if (!jit)
 			launch_fkernel<13>(s, a, grid);
 		break;
@@ -1815,6 +1841,7 @@ void dng_scan_destroy(dng_scan *s)
 	cached_free(s->d_tmpl);
 	cached_free(s->d_fplan);
 	cached_free(s->d_ftmpl);
+	cached_free(s->d_fdict);
 	cached_free(s->d_miss);
 	cached_free(s->d_miss_n);
 	cached_free(s->tab.entries);

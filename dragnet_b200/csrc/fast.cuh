@@ -609,6 +609,34 @@ DNG_PLAN_LOOP
 	return diff == 0;
 }
 
+/* a discrete piece of the key at out + o: u16 length, then byte(k), k < n;
+ * returns the offset after it */
+template <class B>
+DNG_HD u32 fkey_put(u8 *out, u32 o, u32 n, const B &byte)
+{
+	out[o] = (u8)n;
+	out[o + 1] = (u8)(n >> 8);
+#pragma unroll 1
+	for (u32 k = 0; k < n; k++)
+		out[o + 2 + k] = (u8)byte(k);
+	return o + 2 + n;
+}
+
+/* zero padding to a multiple of 8 */
+DNG_HD void fkey_pad(u8 *out, u32 o)
+{
+	while (o & 7)
+		out[o++] = 0;
+}
+
+template <class M>
+struct FPieceBytes {
+	M *m;
+	const FPlan *F;
+	const FPiece *pc;
+	DNG_HD u32 operator()(u32 k) const { return fpiece_byte(*m, *F, *pc, k); }
+};
+
 /* the key's bytes (record.cuh process_metric's encoding), zero padded to a
  * multiple of 8; out has room for F_MAXKEY + 8 */
 template <class M>
@@ -629,15 +657,33 @@ DNG_PLAN_LOOP
 			o += 10;
 			continue;
 		}
-		out[o] = (u8)pc.n;
-		out[o + 1] = (u8)(pc.n >> 8);
-#pragma unroll 1
-		for (u32 k = 0; k < pc.n; k++)
-			out[o + 2 + k] = (u8)fpiece_byte(m, F, pc, k);
-		o += 2 + pc.n;
+		FPieceBytes<M> b;
+		b.m = &m;
+		b.F = &F;
+		b.pc = &pc;
+		o = fkey_put(out, o, pc.n, b);
 	}
-	while (o & 7)
-		out[o++] = 0;
+	fkey_pad(out, o);
+}
+
+struct FDictBytes {
+	const u8 *v;
+	DNG_HD u32 operator()(u32 k) const { return v[k]; }
+};
+
+/* the key of dense counter `idx` (FDict) as fkey_write() writes it: the
+ * dictionary values of its codes; returns the key's length */
+DNG_HD u32 fdense_key(const FDict &D, u32 idx, u8 *out)
+{
+	u32 o = 0;
+	for (u32 j = 0; j < D.ncols; j++) {
+		const u32 c = idx / D.stride[j] % D.n[j];
+		FDictBytes b;
+		b.v = D.val[j][c];
+		o = fkey_put(out, o, D.len[j][c], b);
+	}
+	fkey_pad(out, o);
+	return o;
 }
 
 #ifndef __CUDACC__

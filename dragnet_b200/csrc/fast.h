@@ -69,6 +69,27 @@ struct alignas(16) FPlan {
 };
 
 /*
+ * Dense keys: the values the breakdown columns take in the head of the input,
+ * learned per column (fdict_learn).  A record whose pieces are all in it is
+ * counted at index sum_j code_j * stride[j] of a per-CTA array of u32 counters
+ * instead of being hashed and probed; val[j][c] holds the bytes fkey_write()
+ * would write for code c (String(value), or "null" ...), sorted by bytes.
+ */
+/* (24 bytes: the operation names of a web service's log, "deletepublicstorage"
+ * ..., are longer than 16) */
+enum : int { F_DICT_VALS = 15, F_DICT_BYTES = 24, F_DENSE_MAX = 1024 };
+
+struct alignas(16) FDict {
+	u32 ncols;			/* 0: no dictionary */
+	u32 total;			/* counters: the product of n[] */
+	u32 n[F_MAXCOLS];		/* values of column j */
+	u32 stride[F_MAXCOLS];
+	u8 path[F_MAXCOLS];		/* column j's path (capture row) */
+	u8 len[F_MAXCOLS][F_DICT_VALS];
+	u8 val[F_MAXCOLS][F_DICT_VALS][F_DICT_BYTES];
+};
+
+/*
  * A capture: what the matcher stores for a path of the record at hand.
  * off(12) | len(12) << 12 | type(3) << 24 | flag << 27; off is relative to the
  * record.  flag = VF_ESCAPED for strings, "simple integer" for numbers.
@@ -98,6 +119,16 @@ void fplan_build(const DevPlan &P, FPlan &F);
  * be an F template (a needed path resolves to a container).
  */
 bool fplan_resolve(const DevPlan &P, const TResolved &in, TResolved &out);
+
+/*
+ * The value dictionary of an F plan whose columns are all discrete with a path
+ * source, from the lines of head[0, n) that the F trie `blob` (tmpl_build,
+ * compact) takes to the aggregator (fdict.cpp).  False, and D.ncols = 0, unless
+ * every column has at most F_DICT_VALS values of at most F_DICT_BYTES bytes
+ * covering 99 % of those records, in at most F_DENSE_MAX counters.
+ */
+bool fdict_learn(const FPlan &F, const u8 *blob, const u8 *head, size_t n,
+    FDict &D);
 
 } /* namespace dng */
 

@@ -64,6 +64,9 @@ struct FScanArgs {
 	u32 nchunks, seg;		/* chunks, chunks per segment */
 	u32 final;
 	u32 s1slots, sslots;
+	u32 ndense;			/* dense counters (FDict::total; 0: none),
+					 * rounded up to a multiple of 4 */
+	const FDict *dict;
 	u32 nrows;			/* capture rows (FPlan::nrows) */
 	MissEnt *miss;
 	u32 miss_cap;
@@ -85,11 +88,11 @@ static constexpr u32 FPLAN_SMEM = (sizeof (FPlan) + 127) & ~127u;
  * their stride -- when the tally cache needs the room) */
 template <int NSL>
 static inline size_t fkernel_smem(u32 tmpl_bytes, u32 s1slots, u32 sslots,
-    u32 nrows, u32 nw = DNG_F_NW)
+    u32 nrows, u32 nw = DNG_F_NW, u32 ndense = 0)
 {
 	return FPLAN_SMEM + tmpl_bytes + (size_t)s1slots * sizeof (SSlot1) +
-	    (size_t)sslots * sizeof (SSlot) + (size_t)nrows * DNG_F_NT * 4 +
-	    (size_t)nw * FWarpSmem<NSL>::BYTES;
+	    (size_t)sslots * sizeof (SSlot) + (size_t)ndense * 4 +
+	    (size_t)nrows * DNG_F_NT * 4 + (size_t)nw * FWarpSmem<NSL>::BYTES;
 }
 
 /* mbarrier / TMA helpers on 32-bit shared addresses (no generic pointers to
@@ -249,6 +252,10 @@ extern "C" __device__ void dng_cold_miss(const u8 *data,
     unsigned long long *counters);
 extern "C" __device__ void dng_cold_flush(STab stab, u32 s1slots, u32 sslots,
     const GTable *tab);
+extern "C" __device__ u32 dng_cold_key(FSmem m, const FPlan *F, u32 defmask,
+    STab stab, const GTable *gt, u32 over_sa);
+extern "C" __device__ void dng_cold_dense_flush(u32 dense_sa, const FDict *D,
+    const GTable *gt);
 /*
  * The scan's plan as a CONSTANT of the generated code (jit.cpp writes it out
  * with its initialiser): after link-time optimisation the stage and key code
@@ -257,6 +264,16 @@ extern "C" __device__ void dng_cold_flush(STab stab, u32 s1slots, u32 sslots,
  * rare paths are handed.)
  */
 extern "C" __constant__ const FPlan dng_jplan;
+/*
+ * Dense keys (fast.h FDict), generated with the matcher when the scan learned
+ * a value dictionary: dng_jcode() = the record's dense counter, or ~0u.
+ * dng_jdense (jit.h jit_dense()): 0 no dictionary; bit 0 dense counters, bit 1
+ * keys outside the dictionary hashed inline rather than by a call to
+ * dng_cold_key(), bit 2 lanes with the same counter added up first.
+ */
+extern "C" __constant__ const unsigned dng_jdense;
+extern "C" __device__ unsigned dng_jcode(unsigned ra, unsigned dm,
+    unsigned caps);
 #define fslow_add dng_cold_slow_add
 #define fmiss_inline dng_cold_miss
 #else
@@ -421,6 +438,8 @@ __device__ __forceinline__ void fscan_body(const FScanArgs &a)
 	sp += a.s1slots * sizeof (SSlot1);
 	stab.s = (SSlot *)sp;
 	sp += a.sslots * sizeof (SSlot);
+	const u32 dense_sa = smem_u32(sp);
+	sp += a.ndense * 4;
 	stab.mask1 = a.s1slots - 1;
 	stab.mask = a.sslots - 1;
 	const u32 caps_sa = smem_u32(sp);
@@ -445,8 +464,9 @@ __device__ __forceinline__ void fscan_body(const FScanArgs &a)
 			tdst[i] = tsrc[i];
 		const uint4 z = make_uint4(0, 0, 0, 0);
 		uint4 *tz = (uint4 *)stab.s1;
+		/* (and the dense counters behind it) */
 		const u32 tab_bytes = a.s1slots * (u32)sizeof (SSlot1) +
-		    a.sslots * (u32)sizeof (SSlot);
+		    a.sslots * (u32)sizeof (SSlot) + a.ndense * 4;
 		for (u32 i = tid; i < tab_bytes / 16; i += blockDim.x)
 			tz[i] = z;
 		if (lane == 0)
@@ -708,22 +728,57 @@ __device__ __forceinline__ void fscan_body(const FScanArgs &a)
 						matched = use_tmpl &&
 						    fmatch(m, len, inbuf, defmask);
 					}
+					u32 dc = ~0u;	/* dense counter */
 					if (matched) {
 						double s0, s1;
 						fo = fstage(m, F, defmask, s0, s1);
 						u32 h = 0, klen = 0, slow = 0;
-						if (fo == FO_AGGR && (!fprep(m, F, defmask,
-						    s0, s1, slow) || !fkey_hash(m, F,
-						    defmask, h, klen)))
+						if (fo == FO_AGGR && !fprep(m, F, defmask,
+						    s0, s1, slow))
 							fo = FO_MISS;
+#ifdef DNG_JIT_HOT
+						if (fo == FO_AGGR && (dng_jdense & 1))
+							dc = dng_jcode(m.ra, defmask, m.caps);
+						if (dc != ~0u) {
+							/* (counted below) */
+						} else if (fo == FO_AGGR &&
+						    (dng_jdense & 3) == 1) {
+							/* a key outside the dictionary:
+							 * out of line, so that the loop
+							 * is the dense path's size */
+							if (!dng_cold_key(m, (const FPlan *)smem,
+							    defmask, stab, &a.tab,
+							    smem_u32(&s_drop[15])))
+								fo = FO_MISS;
+						} else
+#endif
 						if (fo == FO_AGGR) {
-							if (slow)
-								atomicAdd(&s_drop[1], 1u);
-							ftally(m, F, (const FPlan *)smem, defmask,
-							    h, klen, stab, a.tab,
-							    smem_u32(&s_drop[15]));
+							if (!fkey_hash(m, F, defmask, h, klen))
+								fo = FO_MISS;
+							else
+								ftally(m, F, (const FPlan *)smem,
+								    defmask, h, klen, stab, a.tab,
+								    smem_u32(&s_drop[15]));
 						}
+						if (fo == FO_AGGR && slow)
+							atomicAdd(&s_drop[1], 1u);
 					}
+#ifdef DNG_JIT_HOT
+					/* dense counters (u32, per launch: like the
+					 * inline tally tier's) */
+					if (dng_jdense & 4) {
+						const u32 peers = __match_any_sync(
+						    0xffffffffu, dc);
+						if (dc != ~0u && !(peers & ltmask))
+							asm volatile("red.shared.add.u32 "
+							    "[%0], %1;" :: "r"(dense_sa +
+							    4 * dc), "r"(__popc(peers))
+							    : "memory");
+					} else if (dc != ~0u) {
+						asm volatile("red.shared.add.u32 [%0], 1;"
+						    :: "r"(dense_sa + 4 * dc) : "memory");
+					}
+#endif
 					const bool done = fo != FO_MISS;
 					ntmpl += __popc(__ballot_sync(0xffffffffu, done));
 					naggr += __popc(__ballot_sync(0xffffffffu,
@@ -783,6 +838,8 @@ __device__ __forceinline__ void fscan_body(const FScanArgs &a)
 
 #ifdef DNG_JIT_HOT
 	__syncthreads();
+	if (a.ndense)
+		dng_cold_dense_flush(dense_sa, a.dict, &a.tab);
 	dng_cold_flush(stab, a.s1slots, a.sslots, &a.tab);
 #else
 	flush_tally(stab, a.s1slots, a.sslots, a.tab);

@@ -244,8 +244,85 @@ static void plan_source(const FPlan &F, std::string &s)
 	s += " }\n};\n";
 }
 
+unsigned jit_dense()
+{
+	const char *v = getenv("DNG_DENSE");
+	return v ? (unsigned)atoi(v) : 1u;
+}
+
+/*
+ * dng_jcode(): the record's dense counter (fast.h FDict), or ~0u when a piece of
+ * its key is not in the dictionary.  The same pieces as fpiece() (fast.cuh):
+ * the record's bytes for a string or a plain integer -- by length, then word by
+ * word against immediates -- and the constant a null / boolean / missing value
+ * stands for.  fprep() has already turned away every other form.
+ */
+static void dense_source(const FDict &D, std::string &s)
+{
+	s += "extern \"C\" __device__ unsigned dng_jcode(unsigned ra, unsigned dm, "
+	    "unsigned caps)\n{\n	JMem m;\n	m.ra = ra;\n	u32 idx = 0;\n";
+	for (u32 j = 0; j < D.ncols; j++) {
+		const u32 p = D.path[j];
+		appendf(s, "	{	/* column %u: path %u, %u values */\n", j, p,
+		    D.n[j]);
+		appendf(s, "	const u32 cw = (dm >> %uu) & 1u ? jlds32(caps + %uu) "
+		    ": 0u;\n", p, p * (u32)F_NT * 4u);
+		s += "	const u32 t = (cw >> 24) & 7u, n = (cw >> 12) & 0xfffu;\n"
+		    "	u32 c = 0xffffffffu;\n"
+		    "	if (t == T_STR || t == T_NUM) {\n"
+		    "		JMem::Cur k = m.cursor(cw & 0xfffu);\n"
+		    "		switch (n) {\n";
+		std::map<u32, std::vector<u32>> bylen;
+		for (u32 c = 0; c < D.n[j]; c++)
+			bylen[D.len[j][c]].push_back(c);
+		for (auto &bl : bylen) {
+			const u32 L = bl.first, nw = (L + 3) / 4;
+			appendf(s, "		case %u: {\n", L);
+			for (u32 w = 0; w < nw; w++) {
+				if (w + 1 == nw && (L & 3))
+					appendf(s, "			const u32 w%u = k.next() & "
+					    "0x%08xu;\n", w, (1u << (8 * (L & 3))) - 1);
+				else
+					appendf(s, "			const u32 w%u = k.next();\n",
+					    w);
+			}
+			bool first = true;
+			for (u32 c : bl.second) {
+				s += first ? "			if (" : "			else if (";
+				first = false;
+				if (nw == 0)
+					s += "true";
+				for (u32 w = 0; w < nw; w++) {
+					u32 lit = 0;
+					for (u32 x = 0; x < 4 && 4 * w + x < L; x++)
+						lit |= (u32)D.val[j][c][4 * w + x] <<
+						    (8 * x);
+					appendf(s, "%sw%u == 0x%08xu", w ? " && " : "",
+					    w, lit);
+				}
+				appendf(s, ")\n				c = %uu;\n",
+				    c * D.stride[j]);
+			}
+			s += "			break;\n		}\n";
+		}
+		s += "		}\n	}\n";
+		/* the constants of fpiece() */
+		static const struct { u32 t; const char *v; } K[] = {
+			{ T_UNDEF, "undefined" }, { T_NULL, "null" },
+			{ T_TRUE, "true" }, { T_FALSE, "false" } };
+		for (auto &kc : K)
+			for (u32 c = 0; c < D.n[j]; c++)
+				if (D.len[j][c] == strlen(kc.v) &&
+				    !memcmp(D.val[j][c], kc.v, D.len[j][c]))
+					appendf(s, "	if (t == %uu)\n		c = %uu;\n",
+					    kc.t, c * D.stride[j]);
+		s += "	if (c == 0xffffffffu)\n		return c;\n	idx += c;\n	}\n";
+	}
+	s += "	return idx;\n}\n";
+}
+
 std::string jit_source(const u8 *blob, size_t bytes, const FPlan *plan,
-    const char *prelude)
+    const char *prelude, const FDict *dict)
 {
 	std::string s;
 	s += "/* generated by libdragnet_gpu (jit.cpp) */\n";
@@ -269,6 +346,22 @@ std::string jit_source(const u8 *blob, size_t bytes, const FPlan *plan,
 	if (plan)
 		plan_source(*plan, s);
 	s.append(dng_fscan_src, (size_t)(dng_fscan_src_end - dng_fscan_src));
+	/*
+	 * Dense keys: the kernel refers to both symbols, so the device build
+	 * always has them -- without a dictionary dng_jdense = 0 and the lookup
+	 * is dead code.  The dictionary is part of the text, hence of the
+	 * kernel cache's key.
+	 */
+	const unsigned mode = jit_dense();
+	const bool dense = dict && dict->ncols && mode;
+	if (plan)
+		appendf(s, "\nextern \"C\" __constant__ const unsigned dng_jdense = "
+		    "%uu;\n", dense ? mode | 1u : 0u);
+	if (dense)
+		dense_source(*dict, s);
+	else if (plan)
+		s += "extern \"C\" __device__ unsigned dng_jcode(unsigned, unsigned, "
+		    "unsigned)\n{\n	return 0xffffffffu;\n}\n";
 	s += "\nextern \"C\" __device__ unsigned dng_jmatch(unsigned ra, "
 	    "unsigned len, unsigned active, unsigned caps)\n{\n"
 	    "	JMem m;\n	m.ra = ra;\n"

@@ -43,9 +43,20 @@ struct JitKernels {
 /* the CUDA source of dng_jmatch() for an F trie blob (tmpl_build, compact)
  * and of the plan constant the kernel is specialised to (null: left out);
  * `prelude` replaces the device definitions the generated code builds on
- * (tests/hostcheck compiles the same code for the host with its own) */
+ * (tests/hostcheck compiles the same code for the host with its own).  With a
+ * value dictionary (dict->ncols != 0) and jit_dense() on, dng_jcode() looks the
+ * record's key up in it (the kernel's dense counters). */
 std::string jit_source(const u8 *blob, size_t bytes, const FPlan *plan,
-    const char *prelude = nullptr);
+    const char *prelude = nullptr, const FDict *dict = nullptr);
+
+/*
+ * Dense keys (fast.h FDict) in the run-time linked kernel: DNG_DENSE, default
+ * 1; 0 turns them off (the hashed tally for every key).  Bits of a value other
+ * than 0 and 1 pick variants: 2 keeps the hashed path for keys outside the
+ * dictionary inline instead of calling it, 4 adds the lanes of a warp that
+ * share a counter together before the shared-memory add.
+ */
+unsigned jit_dense();
 
 /*
  * The kernels for this source on device `dev`, from the cache or built now:
